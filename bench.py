@@ -6,7 +6,7 @@ Workload (BASELINE.json configs[1]): batch = 8 synthetic 64x2048 KITTI-shaped sc
 list/cell-index build + fused SE(3) transform / exact NN / point-to-plane + plane-to-plane loss
 forward and backward to the 3x4 transform, for the whole batch.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 * `value`     : pairs/s with the raw scans already resident in HBM (CUDA events, max over ranks).
                 R input sets are rotated so that a set is re-read only after > L2-size traffic.
@@ -21,6 +21,9 @@ forward and backward to the 3x4 transform, for the whole batch.
                 collective; `cudnn_fp32_ms` / `cudnn_bf16_ms` = the reference's nn.Conv2d stack on the same box (N = 1).
 * `cpu_baseline` / `--impl reference`: the oracle port of the reference's CPU path
                 (oracle/delora_oracle.py: torch-CPU + numpy + scipy cKDTree) on the host cores.
+* `--dump-outputs DIR`: what the last timed step returned on rank 0, `DIR/losses.npy` [8, 8] and
+                `DIR/grad_T.npy` [8, 12] (float32).  The inputs are seeded, so two builds run with the same
+                arguments can be compared output for output.
 Multi-GPU: one process per GPU (torchrun), pairs sharded across ranks, no data-path collective
 (weak scaling: 8 pairs per GPU); barrier + max over ranks for the timing.
 """
@@ -35,6 +38,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
 
 PAIRS_PER_GPU = 8
 H, W, W_RAW = 64, 2048, 2048
@@ -360,12 +364,18 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(K):
-        pipes[i % ROTATE].step()
+        last = pipes[i % ROTATE].step()
     e1.record()
     torch.cuda.synchronize()
     barrier(world)
     t_wall = time.perf_counter() - t_wall
     total_ms = max_over_ranks(e0.elapsed_time(e1), world, device)
+    if args.dump_outputs and rank == 0:
+        # the step's output buffers are overwritten by the passes below: copy them out now
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in zip(("losses", "grad_T"), last):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy().astype(np.float32))
     # per-operator durations (-> `kernels`, `roofline`): K more steps of the same inputs on ONE stream with CUDA events
     # around every operator -- with overlapping sub-batches an operator's duration is not separable
     for i in range(K):
@@ -614,7 +624,13 @@ def main():
                     help="steps of the reference-on-GPU bar (torch nn.Conv2d / cuDNN, fp32 and bf16 autocast; N = 1; 0 = skip)")
     ap.add_argument("--train-batch", type=int, default=16)
     ap.add_argument("--rotate", type=int, default=ROTATE, help="rotating input sets (1 only for profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the losses and transform gradients of the last timed step to DIR/*.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -290,6 +290,32 @@ def test_pair_pipeline_sub_batches_on_streams_are_bit_identical(golden, cuda_lib
     assert float(outs[0][0][:, 3].min()) > 100                          # every pair found correspondences
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path, cuda_lib):
+    """`bench.py --dump-outputs DIR`: the losses and transform gradients of the last timed step, bit for bit what the
+    pipeline returns for the same seeded pairs (one input set, so every step sees pairs 0..7)."""
+    import json
+    import subprocess
+    import sys
+    from delora_b200 import synthetic
+    from delora_b200.pipeline import ScanPairPipeline
+    from helpers import ROOT
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "1", "--rotate", "1",
+                          "--cpu-pairs", "0", "--train-steps", "0", "--stream-frames", "0",
+                          "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, timeout=900, check=True)
+    line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 3
+    losses, grad_t = np.load(tmp_path / "dump" / "losses.npy"), np.load(tmp_path / "dump" / "grad_T.npy")
+    assert losses.dtype == np.float32 and losses.shape == (8, 8) and grad_t.dtype == np.float32 and grad_t.shape == (8, 12)
+    cfg = synthetic.fov_config(h=64, w=2048)
+    pairs = [synthetic.make_pair(i, w_raw=2048) for i in range(8)]
+    n_max = max(max(p[0].shape[1], p[1].shape[1]) for p in pairs)
+    pipe = ScanPairPipeline(8, n_max, 64, 2048, *fov(cfg), device=DEV)
+    pipe.load([p[0] for p in pairs], [p[1] for p in pairs], torch.stack([p[3] for p in pairs]))
+    want_losses, want_grad = pipe.step()
+    assert np.array_equal(losses, want_losses.cpu().numpy()) and np.array_equal(grad_t, want_grad.cpu().numpy())
+    assert float(losses[:, 3].min()) > 1000                               # every pair found correspondences
+
+
 @pytest.mark.parametrize("name", CASES)
 def test_dense_icp_matches_list_icp(name, golden, cuda_lib):
     """The dense-grid kernel (training fast path) against the oracle and against the CSR kernel."""
