@@ -45,6 +45,7 @@ SIGNATURES = {
     "delora_conv2d_fprop_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                          c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "delora_conv_select_kernel": (c_int, [c_int]),
+    "delora_conv2d_dgrad_supported": (c_int, [c_int, c_int, c_int, c_int, c_int]),
     "delora_conv2d_dgrad_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                          c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "delora_conv2d_wgrad_scratch_floats": (c_i64, [c_int, c_int, c_int, c_int, c_int, c_int]),

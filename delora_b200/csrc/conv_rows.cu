@@ -566,6 +566,14 @@ int conv_rows_launch(const void* x, const void* w, const void* residual, const v
 
 using namespace delora;
 
+// the shape conditions of delora_conv2d_dgrad_bf16 (forward Cin / Cout); they depend on the pair setting through
+// rows_pixm, so callers ask here instead of restating them
+extern "C" int delora_conv2d_dgrad_supported(int Cin, int Cout, int Win, int stride_h, int stride_w) {
+    if (!((stride_h == 1 || stride_h == 2) && (stride_w == 1 || stride_w == 2) && Win >= 1)) return 0;
+    if (stride_w == 2 && Win % 2 != 0) return 0;
+    return conv_rows_eligible(Cout, Cin, 3, (Win + stride_w - 1) / stride_w) ? 1 : 0;
+}
+
 extern "C" int delora_conv2d_dgrad_bf16(const void* dz, const void* w_flip, const void* residual, const void* saved,
                                         void* dx, int B, int Hin, int Win, int Cin, int Cout, int stride_h, int stride_w,
                                         int act, int residual_strided, void* stream) {
@@ -575,9 +583,9 @@ extern "C" int delora_conv2d_dgrad_bf16(const void* dz, const void* w_flip, cons
     DELORA_CHECK_ARG((stride_h == 1 || stride_h == 2) && (stride_w == 1 || stride_w == 2) && Hin >= 1 && Win >= 1,
                      "delora_conv2d_dgrad_bf16: stride (%d,%d) unsupported", stride_h, stride_w);
     DELORA_CHECK_ARG(stride_w == 1 || Win % 2 == 0, "delora_conv2d_dgrad_bf16: stride_w = 2 needs an even Win (got %d)", Win);
-    DELORA_CHECK_ARG(conv_rows_eligible(Cout, Cin, 3, (Win + stride_w - 1) / stride_w),
-                     "delora_conv2d_dgrad_bf16: needs Cout %% 64 == 0 and Cin %% 128 == 0 (or Cin = 64 / 128 with at least "
-                     "128 columns per phase); got Cin=%d, Cout=%d, Win=%d", Cin, Cout, Win);
+    DELORA_CHECK_ARG(delora_conv2d_dgrad_supported(Cin, Cout, Win, stride_h, stride_w),
+                     "delora_conv2d_dgrad_bf16: needs Cout %% 64 == 0 and Cin %% 128 == 0 (or Cin = 64 with at least "
+                     "128 columns per phase and CTA pairs enabled); got Cin=%d, Cout=%d, Win=%d", Cin, Cout, Win);
     return conv_rows_launch(dz, w_flip, residual, saved, dx, B, Hin, Win, Cout, Cin, 3, stride_h, stride_w, act,
                             (cudaStream_t)stream, residual_strided);
 }

@@ -882,6 +882,7 @@ static const TensorMaps* get_maps(const void* x, const void* w, int B, int Hin, 
 namespace delora {
 bool conv_rows_eligible(int Cin, int Cout, int ksize, int Wg);
 void rows_set_pairs(int on);
+bool rows_use_pairs();
 bool wgrad2_eligible(int Cin, int Cout, int ksize, int stride_h, int stride_w);
 int64_t wgrad2_scratch_floats(int B, int Hout, int Wout, int Cin, int Cout, int sw);
 int wgrad2_launch(const void* x, const void* dz, float* dw, float* scratch, int B, int Hin, int Win, int Cin, int Cin_true,
@@ -900,7 +901,7 @@ static bool use_conv_rows() {
 using namespace delora;
 
 extern "C" int delora_conv_select_kernel(int rows_kernel) {
-    const int prev = use_conv_rows() ? 1 : 0;
+    const int prev = !use_conv_rows() ? 0 : (rows_use_pairs() ? 1 : 2);
     if (rows_kernel == 0 || rows_kernel == 1) { g_conv_rows = rows_kernel; rows_set_pairs(1); }
     if (rows_kernel == 2) { g_conv_rows = 1; rows_set_pairs(0); }          // row-block kernel, single CTAs only
     return prev;

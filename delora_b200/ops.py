@@ -331,10 +331,9 @@ def conv2d_fprop(x, weight, hin, win, ksize, stride, act=ACT_NONE, residual=None
 
 
 def conv2d_dgrad_eligible(cin, cout, win, stride):
-    """Can delora_conv2d_dgrad_bf16 (phase-decomposed data gradient) take this layer?"""
-    wg = (win + stride[1] - 1) // stride[1]
-    return (cout % 64 == 0 and (cin % 128 == 0 or (cin == 64 and wg >= 128))
-            and (stride[1] == 1 or win % 2 == 0))
+    """Can delora_conv2d_dgrad_bf16 (phase-decomposed data gradient) take this layer?  The library answers: the
+    conditions depend on the kernel selection (delora_conv_select_kernel(2) / DELORA_CONV_PAIRS=0 rule out Cin = 64)."""
+    return bool(_lib.lib().delora_conv2d_dgrad_supported(int(cin), int(cout), int(win), int(stride[0]), int(stride[1])))
 
 
 def conv2d_dgrad(dz, w_flip, hin, win, stride, act=ACT_NONE, residual=None, out=None, saved=None,

@@ -250,7 +250,9 @@ int delora_conv2d_fprop_bf16(const void* x, const void* w, const void* residual,
                              void* stream);
 /* Measurement switch: 1 (default) lets delora_conv2d_fprop_bf16 use the row-block kernel (csrc/conv_rows.cu) for
  * stride-1 layers with Cout % 128 == 0, 0 keeps every layer on the tap-per-TMA kernel (csrc/conv_tc.cu); any other
- * value only queries.  Returns the previous setting.  Same effect as the environment variable DELORA_CONV_ROWS=0. */
+ * value only queries.  2 keeps the row-block kernel but runs it on single CTAs only (no CTA pairs; same effect as
+ * DELORA_CONV_PAIRS=0).  Returns the previous setting (0, 1 or 2).  0 has the same effect as the environment variable
+ * DELORA_CONV_ROWS=0. */
 int delora_conv_select_kernel(int rows_kernel);
 /* Data gradient of a 3x3 convolution of stride (stride_h, stride_w) in {1,2}^2 -- autograd's backward of the same
  * nn.Conv2d layers (src/models/resnet_modified.py:126-134) w.r.t. their input -- by PHASE DECOMPOSITION: every
@@ -261,11 +263,14 @@ int delora_conv_select_kernel(int rows_kernel);
  * residual_strided = 1: `residual` is [B,Hout+2,Wout+2,Cin] instead and is added at the input pixels
  * (stride_h * h, stride_w * w) only -- the data gradient of the block's 1x1 strided downsample (:134), which never
  * reaches the other pixels (replaces a zero-upsampled copy of it).
- * Needs Cout % 64 == 0, Cin % 128 == 0 (or Cin = 64 with >= 128 columns per phase) and, for stride_w = 2, an even Win (an odd circular width mixes the phases at
+ * Needs Cout % 64 == 0, Cin % 128 == 0 (or Cin = 64 with >= 128 columns per phase and CTA pairs enabled) and, for stride_w = 2, an even Win (an odd circular width mixes the phases at
  * the seam: use delora_zero_upsample_nhwc_bf16 + delora_conv2d_fprop_bf16 there). */
 int delora_conv2d_dgrad_bf16(const void* dz, const void* w_flip, const void* residual, const void* saved, void* dx,
                              int B, int Hin, int Win, int Cin, int Cout, int stride_h, int stride_w, int act,
                              int residual_strided, void* stream);
+/* 1 if delora_conv2d_dgrad_bf16 takes this layer (forward Cin / Cout, input width, stride) under the current kernel
+ * selection, else 0.  No GPU work; the answer changes with delora_conv_select_kernel(2) (Cin = 64 needs CTA pairs). */
+int delora_conv2d_dgrad_supported(int Cin, int Cout, int Win, int stride_h, int stride_w);
 /* Weight gradient of the same convolution on tcgen05 (split-K over pixels, deterministic reduction):
  * x [B,Hin+2,Win+2,Cin] padded NHWC bf16 (the layer input), dz [B,Hout+2,Wout+2,Cout] padded NHWC bf16
  * (gradient w.r.t. the pre-activation output) -> dw [Cout, Cin_true, k, k] fp32 (torch layout; Cin_true <= Cin
